@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU arithmetic on the host cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's tokens and latents to DIR/*.npy
 
 One "step" = one pass of the hot path over one batch: encode (16-block Q-Former + fused VQ -> 512 tokens) followed by
 the 50-step rectified-flow decode of those tokens (24-layer MMDiT), 256x256 images, no VAE (latent boundary; SURVEY 8f).
@@ -45,6 +46,7 @@ METRIC = "images/sec encode+50-step decode, 256x256/512-tok"
 UNIT = "images/s"
 BATCH = 64
 DECODE_STEPS = 50
+DUMP_BYTES = 64 << 20
 
 
 def peaks():
@@ -244,6 +246,22 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------ GPU arm
+def dump_outputs(path, outputs):
+    """Write what a caller of the timed step receives (token ids [B, K], latents [B, 16, 32, 32]) as DIR/<name>.npy: ids as
+    float64 (exact), latents as float32.  Above DUMP_BYTES in all, a fixed seeded sample of images is written instead, so two
+    builds run with the same arguments can be compared file for file."""
+    import numpy as np
+    arrays = {"tokens": outputs["tokens"].cpu().double().numpy(), "latents": outputs["latents"].cpu().float().numpy()}
+    B = arrays["tokens"].shape[0]
+    per_image = sum(a[0].nbytes for a in arrays.values())
+    if per_image * B > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(B, DUMP_BYTES // per_image, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_extras(args, eng, dev, x0, noise, timed):
     """Sub-records for BASELINE configs 2 and 4 and the fp32-faithful mode (see the module docstring).  `eng` is the
     headline engine (still alive); every other engine is created here and closed before the next one."""
@@ -405,13 +423,14 @@ def run_gpu(args):
     x0_h, noise_h = x0.cpu().pin_memory(), noise.cpu().pin_memory()
     tok_h = torch.empty(B, d.K, dtype=torch.int64).pin_memory()
     out_h = torch.empty_like(noise_h).pin_memory()
+    last = {}                                       # outputs of the latest step_device call (kept for --dump-outputs)
 
     def step_device():
         tok = eng.encode(x0)
         n = eng.last_launch_count
         if world > 1:
             gather_tokens(tok, B * world)           # the path's only exchange: [B,512] int64 per rank over NVLink
-        eng.decode(tok, noise)
+        last["tokens"], last["latents"] = tok, eng.decode(tok, noise)
         return n + eng.last_launch_count
 
     def step_host():
@@ -449,6 +468,9 @@ def run_gpu(args):
         sampler.start()
     ms, launches = timed(step_device, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
+    last.clear()
     value = B * world * args.steps / (ms / 1000.0)
     # ---- end to end through the host-buffer entry points
     step_host()
@@ -532,7 +554,13 @@ def main():
     ap.add_argument("--batch", type=int, default=BATCH)
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extra", action="store_true", help="skip the sub-records of the other BASELINE configs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the tokens and latents of the last timed step as DIR/tokens.npy and DIR/latents.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs applies to the CUDA path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
         return

@@ -181,9 +181,13 @@ def gen_pixels_tiny():
     save("tiny_pixels", pixels=ref_pixels(vae, torch.from_numpy(g["pred_x0"])))
 
 
+RENDERER_PIXEL_STRIDE = 2
+
+
 def gen_pixels_full():
     """Full geometry, B = 1: reference latents of tests/golden/full_decode.npz and full_renderer.npz through the
-    full-size (ch = 128) reference SDVAE -> [1,3,256,256] pixels in [0,1]."""
+    full-size (ch = 128) reference SDVAE -> [1,3,256,256] pixels in [0,1].  The renderer's image is kept at every second row
+    and column (RENDERER_PIXEL_STRIDE): two full fp32 images do not compress below 1 MB."""
     vae = ref_vae(128)
     g = np.load(os.path.join(GOLD, "full_decode.npz"))
     gr = np.load(os.path.join(GOLD, "full_renderer.npz"))
@@ -191,7 +195,35 @@ def gen_pixels_full():
     px = ref_pixels(vae, torch.from_numpy(g["pred_x0"]))
     pr = ref_pixels(vae, torch.from_numpy(gr["pred_x0"]))
     print(f"SDVAE decode of 2 images: {time.time() - t0:.1f}s; in-range fraction {float(((px > 0) & (px < 1)).float().mean()):.3f}")
-    save("full_pixels", pixels=px, renderer_pixels=pr)
+    s = RENDERER_PIXEL_STRIDE
+    save("full_pixels", pixels=px, renderer_pixels=pr[..., ::s, ::s])
+
+
+def gen_tiny_module():
+    """The reference's own modules built on the TINY geometry: the name and shape of every entry of their state dict (the
+    contract synth.state_dict_spec must meet) and the encoder's tokens and quantised outputs for two seeded latents."""
+    import json
+    dims = C.TINY
+    pipe, _ = build(dims, tag="tinymodule")
+    shapes = {k: list(v.shape) for k, v in pipe.model.state_dict().items()}
+    x0 = synth.synth_tensor("live.x0", (2, dims.in_channels, dims.latent, dims.latent), "emb", 1.0)
+    with torch.no_grad():
+        outs_q, tokens = pipe.model.encoder(x0, d=None)
+    save("tiny_module", state_dict_shapes=np.array(json.dumps(shapes)), tokens=tokens, outs_q=outs_q)
+
+
+def gen_boundary():
+    """The reference's boundary helpers (SelftokPipeline.py:85-97,135-137; sd3/sd3_impls.py:133-144) on seeded inputs:
+    NormalizeToTensor of an 8-bit image, norm_ip, and SD3LatentFormat.process_in / process_out."""
+    ref_loader.import_reference()
+    from mimogpt.infer import SelftokPipeline as SP
+    from mimogpt.models.selftok.sd3.sd3_impls import SD3LatentFormat
+    img = np.random.RandomState(0).randint(0, 256, size=(24, 40, 3)).astype(np.uint8)
+    y = torch.tensor([-3.0, -1.0, 0.0, 0.5, 1.0, 2.0])
+    SP.norm_ip(y, -1, 1)
+    lat = synth.synth_tensor("golden.boundary.lat", (2, 16, 4, 4), "emb", 1.0)
+    save("boundary", normalized=SP.NormalizeToTensor()(img), norm_ip=y, process_in=SD3LatentFormat().process_in(lat),
+         process_out=SD3LatentFormat().process_out(lat))
 
 
 def save(name, **arrs):
@@ -401,5 +433,9 @@ if __name__ == "__main__":
             gen_pixels_tiny()
         elif w == "full_pixels":
             gen_pixels_full()
+        elif w == "tiny_module":
+            gen_tiny_module()
+        elif w == "boundary":
+            gen_boundary()
         else:
             raise SystemExit(f"unknown target {w}")

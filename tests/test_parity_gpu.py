@@ -374,6 +374,8 @@ def test_full_pixel_gate(full_engine, gold):
 
 
 def test_full_renderer_pixel_gate(gold):
+    """The pixel gate of the renderer pass; the fixture keeps the reference's pixels at every second row and column
+    (oracle/gen_golden.py RENDERER_PIXEL_STRIDE), and ours and the target are compared at the same positions."""
     import vae_oracle as V
     from selftoktokenizer_b200.capi import Engine
     gr, ge, gp = gold("full_renderer"), gold("full_encode"), gold("full_pixels")
@@ -387,7 +389,9 @@ def test_full_renderer_pixel_gate(gold):
         px = V.images_from_latents(vsd, r).numpy()
         x0 = synth.synth_tensor("golden.full.x0", (2, d.in_channels, d.latent, d.latent), "emb", 1.0)[:1]
         gt = V.images_from_latents(vsd, x0).numpy()
-    _pixel_gate(px, gp["renderer_pixels"], gt, "full renderer bf16x3")
+    s = 2
+    assert gp["renderer_pixels"].shape == px[..., ::s, ::s].shape
+    _pixel_gate(px[..., ::s, ::s], gp["renderer_pixels"], gt[..., ::s, ::s], "full renderer bf16x3")
 
 
 @pytest.mark.parametrize("fixture,stress", [("mid", False), ("mid_stress", True)])
