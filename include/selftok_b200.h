@@ -143,6 +143,22 @@ int selftok_dit_velocity(selftok_handle_t h, const int64_t* tokens_dev, const fl
 /* renderer handles only: tokens_dev [B,K] -> pred_x0 [B,C,latent,latent]. */
 int selftok_render(selftok_handle_t h, const int64_t* tokens_dev, int B, float* x0_out_dev, void* stream);
 
+/* ---- decode from a token prefix: image b from its first n_b tokens (the reference's super_mask[b] = arange(K) < n_b,
+ * sd3/rectified_flow.py:182,227-228; renderer: mask[b], sd3/mmdit.py:1511,1529).  At step i image b sees the context tokens
+ * < min(k_i + 1, n_b); ids at positions >= n_b are never read (not range-checked, may be -1); n_b = K for every image gives
+ * the result of the entry point without a prefix.  Per-image results depend only on that image and max_b n_b.
+ * n_tokens_host: int32 [B] host array, 1 <= n_b <= K (read before the call returns; the host needs max n to shape launches);
+ * any other value returns SELFTOK_ERR_BAD_ARG and launches nothing.
+ * cfg_scale == 1: plain sampler (captured graphs keyed by batch, steps and the per-step context rows, which every
+ * max n >= k_0 + 1 shares); otherwise the guided sampler with the prefix applied to its conditional branch. */
+int selftok_decode_prefix(selftok_handle_t h, const int64_t* tokens_dev, const int32_t* n_tokens_host, const float* noise_dev,
+                          int B, int steps, float cfg_scale, float* x0_out_dev, void* stream);
+int selftok_render_prefix(selftok_handle_t h, const int64_t* tokens_dev, const int32_t* n_tokens_host, int B,
+                          float* x0_out_dev, void* stream);
+/* testing / bisecting entry, like selftok_dit_velocity */
+int selftok_dit_velocity_prefix(selftok_handle_t h, const int64_t* tokens_dev, const int32_t* n_tokens_host, const float* x_dev,
+                                int B, int step, float* v_out_dev, void* stream);
+
 /* ---- hot path, host buffers (what SelftokPipeline's numpy-in / tensor-out API maps to; H2D and D2H copies are
  * inside the call, on `stream`, followed by a stream synchronize) --------------------------------------------- */
 int selftok_encode_host(selftok_handle_t h, const float* x0_host, int B, int64_t* tokens_host, void* stream);

@@ -24,6 +24,7 @@ SYMBOLS = [
     "selftok_create", "selftok_destroy", "selftok_last_error", "selftok_version", "selftok_load_tensor",
     "selftok_set_schedule", "selftok_finalize", "selftok_export_packed", "selftok_import_packed", "selftok_encode", "selftok_vq_argmax", "selftok_lookup",
     "selftok_set_cfg_schedule", "selftok_decode", "selftok_decode_cfg", "selftok_dit_velocity", "selftok_render", "selftok_encode_host", "selftok_decode_host",
+    "selftok_decode_prefix", "selftok_render_prefix", "selftok_dit_velocity_prefix",
     "selftok_render_host", "selftok_id_errors", "selftok_workspace_bytes", "selftok_set_workspace", "selftok_last_launch_count", "selftok_device_bytes", "selftok_set_use_graph",
     "selftok_set_profile", "selftok_get_profile", "selftok_k_linear_f32", "selftok_k_linear_tc", "selftok_k_set_gemm_ctas", "selftok_k_ln_mod_f32", "selftok_k_attention_f32",
     "selftok_k_attention_tc",
@@ -73,6 +74,9 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
     lib.selftok_decode_cfg.argtypes = [vp, vp, vp, i32, i32, C.c_float, vp, vp]
     lib.selftok_dit_velocity.argtypes = [vp, vp, vp, i32, i32, vp, vp]
     lib.selftok_render.argtypes = [vp, vp, i32, vp, vp]
+    lib.selftok_decode_prefix.argtypes = [vp, vp, vp, vp, i32, i32, C.c_float, vp, vp]
+    lib.selftok_render_prefix.argtypes = [vp, vp, vp, i32, vp, vp]
+    lib.selftok_dit_velocity_prefix.argtypes = [vp, vp, vp, vp, i32, i32, vp, vp]
     lib.selftok_encode_host.argtypes = [vp, vp, i32, vp, vp]
     lib.selftok_decode_host.argtypes = [vp, vp, vp, i32, i32, vp, vp]
     lib.selftok_render_host.argtypes = [vp, vp, i32, vp, vp]
@@ -262,17 +266,35 @@ class Engine:
             raise SelftokError(f"{what}: expected [B, {want[0]}, {want[1]}, {want[2]}] latents for this engine "
                                f"(image side {8 * d.latent}), got {tuple(x.shape)}")
 
-    def _check_tokens(self, tokens: torch.Tensor, what: str, batch: Optional[int] = None, is_output: bool = False) -> None:
+    def _check_tokens(self, tokens: torch.Tensor, what: str, batch: Optional[int] = None, is_output: bool = False,
+                      n_tokens: Optional[torch.Tensor] = None) -> None:
         if tokens.dim() != 2 or tokens.shape[1] != self.dims.K or tokens.shape[0] < 1:
             raise SelftokError(f"{what}: expected [B, {self.dims.K}] token ids, got {tuple(tokens.shape)}")
         if batch is not None and tokens.shape[0] != batch:
             raise SelftokError(f"{what}: {tokens.shape[0]} token rows for a batch of {batch}")
         if not tokens.is_cuda and not is_output:
             # ids outside the codebook are an error in the reference (`codebook[idx]` raises).  Host tensors are checked here
-            # for free; device tensors are checked by the kernel (NaN rows + counter, see `id_errors`).
+            # for free; device tensors are checked by the kernel (NaN rows + counter, see `id_errors`).  With a token prefix
+            # only the ids inside each image's prefix are read.
+            if n_tokens is not None:
+                tokens = tokens[torch.arange(self.dims.K)[None, :] < n_tokens[:, None].long()]
+                if tokens.numel() == 0:
+                    return
             lo, hi = int(tokens.min()), int(tokens.max())
             if lo < 0 or hi >= self.dims.codebook_size:
                 raise SelftokError(f"{what}: token id out of range [0, {self.dims.codebook_size}): min {lo}, max {hi}")
+
+    def _n_tokens(self, n_tokens, B: int) -> Optional[torch.Tensor]:
+        """Per-image prefix lengths (an int for the whole batch, or B values) -> int32 host tensor [B]; None stays None.
+        The range [1, K] is checked by the library; values are clamped to [-1, K + 1] first only so that they fit int32."""
+        if n_tokens is None:
+            return None
+        n = torch.as_tensor(n_tokens, dtype=torch.int64).cpu().reshape(-1)
+        if n.numel() == 1:
+            n = n.expand(B)
+        if n.numel() != B:
+            raise SelftokError(f"n_tokens: {n.numel()} prefix lengths for a batch of {B}")
+        return n.clamp(-1, self.dims.K + 1).to(torch.int32).contiguous()
 
     def id_errors(self) -> int:
         """Synchronises and returns how many out-of-range token ids the device lookups saw since the last query."""
@@ -314,48 +336,71 @@ class Engine:
             check(self.lib.selftok_lookup(self.h, tokens.data_ptr(), B, out.data_ptr(), _stream_ptr(self.device)))
         return out
 
-    def decode(self, tokens: torch.Tensor, noise: torch.Tensor, steps: Optional[int] = None) -> torch.Tensor:
+    # n_tokens (decode, decode_cfg, dit_velocity, render): decode image b from its first n_tokens[b] tokens only -- an int for
+    # the whole batch or B values in [1, K]; ids after each prefix are never read.  None: all K tokens (the plain entry points).
+    def decode(self, tokens: torch.Tensor, noise: torch.Tensor, steps: Optional[int] = None, n_tokens=None) -> torch.Tensor:
         self._check_latent(noise, "decode (noise)")
-        self._check_tokens(tokens, "decode", noise.shape[0])
+        n = self._n_tokens(n_tokens, noise.shape[0])
+        self._check_tokens(tokens, "decode", noise.shape[0], n_tokens=n)
         tokens = self._dev(tokens, torch.int64)
         noise = self._dev(noise, torch.float32)
         B = tokens.shape[0]
         out = torch.empty_like(noise)
         with torch.cuda.device(self.device):
-            check(self.lib.selftok_decode(self.h, tokens.data_ptr(), noise.data_ptr(), B, steps or self.steps,
-                                          out.data_ptr(), _stream_ptr(self.device)))
+            if n is None:
+                check(self.lib.selftok_decode(self.h, tokens.data_ptr(), noise.data_ptr(), B, steps or self.steps,
+                                              out.data_ptr(), _stream_ptr(self.device)))
+            else:
+                check(self.lib.selftok_decode_prefix(self.h, tokens.data_ptr(), n.data_ptr(), noise.data_ptr(), B, steps or self.steps,
+                                                     1.0, out.data_ptr(), _stream_ptr(self.device)))
         return out
 
-    def decode_cfg(self, tokens: torch.Tensor, noise: torch.Tensor, cfg_scale: float, steps: Optional[int] = None) -> torch.Tensor:
+    def decode_cfg(self, tokens: torch.Tensor, noise: torch.Tensor, cfg_scale: float, steps: Optional[int] = None,
+                   n_tokens=None) -> torch.Tensor:
         """Guided sampler: the reference's p_sample_loop(..., uncond_scale=cfg_scale) (rectified_flow.py:280-289)."""
         self._check_latent(noise, "decode_cfg (noise)")
-        self._check_tokens(tokens, "decode_cfg", noise.shape[0])
+        n = self._n_tokens(n_tokens, noise.shape[0])
+        self._check_tokens(tokens, "decode_cfg", noise.shape[0], n_tokens=n)
         tokens = self._dev(tokens, torch.int64)
         noise = self._dev(noise, torch.float32)
         out = torch.empty_like(noise)
         with torch.cuda.device(self.device):
-            check(self.lib.selftok_decode_cfg(self.h, tokens.data_ptr(), noise.data_ptr(), tokens.shape[0], steps or self.steps,
-                                              float(cfg_scale), out.data_ptr(), _stream_ptr(self.device)))
+            if n is None:
+                check(self.lib.selftok_decode_cfg(self.h, tokens.data_ptr(), noise.data_ptr(), tokens.shape[0], steps or self.steps,
+                                                  float(cfg_scale), out.data_ptr(), _stream_ptr(self.device)))
+            else:
+                check(self.lib.selftok_decode_prefix(self.h, tokens.data_ptr(), n.data_ptr(), noise.data_ptr(), tokens.shape[0],
+                                                     steps or self.steps, float(cfg_scale), out.data_ptr(), _stream_ptr(self.device)))
         return out
 
-    def dit_velocity(self, tokens: torch.Tensor, x: torch.Tensor, step: int) -> torch.Tensor:
+    def dit_velocity(self, tokens: torch.Tensor, x: torch.Tensor, step: int, n_tokens=None) -> torch.Tensor:
         self._check_latent(x, "dit_velocity")
-        self._check_tokens(tokens, "dit_velocity", x.shape[0])
+        n = self._n_tokens(n_tokens, x.shape[0])
+        self._check_tokens(tokens, "dit_velocity", x.shape[0], n_tokens=n)
         tokens = self._dev(tokens, torch.int64)
         x = self._dev(x, torch.float32)
         out = torch.empty_like(x)
         with torch.cuda.device(self.device):
-            check(self.lib.selftok_dit_velocity(self.h, tokens.data_ptr(), x.data_ptr(), tokens.shape[0], step,
-                                                out.data_ptr(), _stream_ptr(self.device)))
+            if n is None:
+                check(self.lib.selftok_dit_velocity(self.h, tokens.data_ptr(), x.data_ptr(), tokens.shape[0], step,
+                                                    out.data_ptr(), _stream_ptr(self.device)))
+            else:
+                check(self.lib.selftok_dit_velocity_prefix(self.h, tokens.data_ptr(), n.data_ptr(), x.data_ptr(), tokens.shape[0], step,
+                                                           out.data_ptr(), _stream_ptr(self.device)))
         return out
 
-    def render(self, tokens: torch.Tensor) -> torch.Tensor:
-        self._check_tokens(tokens, "render")
+    def render(self, tokens: torch.Tensor, n_tokens=None) -> torch.Tensor:
+        n = self._n_tokens(n_tokens, tokens.shape[0]) if tokens.dim() == 2 else None
+        self._check_tokens(tokens, "render", n_tokens=n)
         tokens = self._dev(tokens, torch.int64)
         d = self.dims
         out = torch.empty(tokens.shape[0], d.in_channels, d.latent, d.latent, dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.device):
-            check(self.lib.selftok_render(self.h, tokens.data_ptr(), tokens.shape[0], out.data_ptr(), _stream_ptr(self.device)))
+            if n is None:
+                check(self.lib.selftok_render(self.h, tokens.data_ptr(), tokens.shape[0], out.data_ptr(), _stream_ptr(self.device)))
+            else:
+                check(self.lib.selftok_render_prefix(self.h, tokens.data_ptr(), n.data_ptr(), tokens.shape[0], out.data_ptr(),
+                                                     _stream_ptr(self.device)))
         return out
 
     # ------------------------------------------------------------------ hot path (host buffers; copies inside the call)

@@ -26,6 +26,8 @@
 //
 // Contract (sd3/mmdit.py:521-531, sd3/other_impls.py:37-45): dense non-causal attention over the joint
 // [context prefix ; image] sequence; rows < ctx_rows only see keys < ctx_keys (renderer rule, mmdit.py:1581).
+// PREFIX variant (decode from a token prefix): image b also ignores the context keys [min(kc, n_ctx[b]), kc), where kc is the
+// number of context rows of the launch (image keys start there); key tiles wholly inside that hole are skipped by every role.
 #include "common.cuh"
 #include "kernels.h"
 
@@ -233,9 +235,23 @@ struct Attn5Params {
   AttnOut out;
   int B, S, H, ctx_rows, ctx_keys, fp16;
   float scale_log2e;
+  const int32_t* n_ctx;         // PREFIX: visible context tokens per image [B]
+  int kc;                       // PREFIX: context rows of the joint sequence
 };
 
-template <bool FP16, int NSPLIT>
+// PREFIX tile map of one item whose image sees context keys [0, hole0) and image keys [kc, S): the n1 key tiles from key 0,
+// then the tiles from h1 on (those in between lie wholly inside the hole); kmax_cta = the item's key limit (kc for an item of
+// context rows only)
+__device__ __forceinline__ int prefix_tiles(int kmax_cta, int hole0, int kc) {
+  const int n1 = (min(hole0, kmax_cta) + BKV - 1) / BKV, h1 = max(n1, kc / BKV);
+  return n1 + (kmax_cta > kc ? max(0, (kmax_cta + BKV - 1) / BKV - h1) : 0);
+}
+__device__ __forceinline__ int prefix_key0(int j, int hole0, int kc) {        // first key of the item's j-th tile
+  const int n1 = (hole0 + BKV - 1) / BKV;
+  return (j < n1 ? j : max(n1, kc / BKV) + (j - n1)) * BKV;
+}
+
+template <bool FP16, int NSPLIT, bool PREFIX>
 __global__ void __launch_bounds__(NUM_THREADS, A5<NSPLIT>::MIN_CTAS)
 attention_tc5_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_kv,
                      const __grid_constant__ CUtensorMap map_q_lo, const __grid_constant__ CUtensorMap map_kv_lo, const Attn5Params p) {
@@ -273,10 +289,15 @@ attention_tc5_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
   // warps finish the current one (no per-item prologue bubble).
   const int nq = (S + BQ - 1) / BQ;
   const int n_items = nq * p.H * p.B;
+  // PREFIX: the item's image sees context keys [0, kcb) and image keys [kc, S); its tile sequence is the n1 tiles from key 0
+  // followed by the tiles from h1 on (the tiles in between lie wholly inside the hole)
   auto item_tiles = [&](int qt) {
     const int kmax_cta = ((qt + 1) * BQ <= p.ctx_rows) ? p.ctx_keys : S;  // every row of the tile is a context row
     return (kmax_cta + BKV - 1) / BKV;
   };
+#define PREFIX_HOLE(item) min(p.kc, __ldg(p.n_ctx + (item) / (nq * p.H)))
+#define PREFIX_TILES(item) \
+  prefix_tiles((((item) % nq + 1) * BQ <= p.ctx_rows) ? p.ctx_keys : S, PREFIX_HOLE(item), p.kc)
 
   if (warp == 1 && lane == 0) {
     for (int i = 0; i < 2; ++i) { mbar_init(q_full(i), 1); mbar_init(q_empty(i), 1); }
@@ -302,13 +323,13 @@ attention_tc5_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
   struct Cur { int item, n, j, nt; };
   auto cur_first = [&]() {
     Cur c{(int)blockIdx.x, 0, 0, 0};
-    c.nt = c.item < n_items ? item_tiles(c.item % nq) : 0;
+    c.nt = c.item < n_items ? (PREFIX ? PREFIX_TILES(c.item) : item_tiles(c.item % nq)) : 0;
     return c;
   };
   auto cur_next = [&](Cur& c) {
     if (++c.j == c.nt) {
       c.item += gridDim.x; ++c.n; c.j = 0;
-      c.nt = c.item < n_items ? item_tiles(c.item % nq) : 0;
+      c.nt = c.item < n_items ? (PREFIX ? PREFIX_TILES(c.item) : item_tiles(c.item % nq)) : 0;
     }
   };
   Cur cq = cur_first();
@@ -355,11 +376,12 @@ attention_tc5_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
         mbar_wait(kv_empty(st), ((g / KV_STAGES) & 1) ^ 1);
         const uint32_t ks = kv_s + st * C::KV_STAGE;
         mbar_expect_tx(kv_full(st), C::KV_STAGE);
-        tma_load_2d(ks, &map_kv, kv_full(st), (p.H + h) * HD, row0 + j * BKV);
-        tma_load_2d(ks + KV_TILE_BYTES, &map_kv, kv_full(st), (2 * p.H + h) * HD, row0 + j * BKV);
+        const int key0 = PREFIX ? prefix_key0(j, PREFIX_HOLE(item), p.kc) : j * BKV;
+        tma_load_2d(ks, &map_kv, kv_full(st), (p.H + h) * HD, row0 + key0);
+        tma_load_2d(ks + KV_TILE_BYTES, &map_kv, kv_full(st), (2 * p.H + h) * HD, row0 + key0);
         if (NSPLIT == 3) {
-          tma_load_2d(ks + 2 * KV_TILE_BYTES, &map_kv_lo, kv_full(st), (p.H + h) * HD, row0 + j * BKV);
-          tma_load_2d(ks + 3 * KV_TILE_BYTES, &map_kv_lo, kv_full(st), (2 * p.H + h) * HD, row0 + j * BKV);
+          tma_load_2d(ks + 2 * KV_TILE_BYTES, &map_kv_lo, kv_full(st), (p.H + h) * HD, row0 + key0);
+          tma_load_2d(ks + 3 * KV_TILE_BYTES, &map_kv_lo, kv_full(st), (2 * p.H + h) * HD, row0 + key0);
         }
       };
       if (SPLIT_ISSUE) {
@@ -393,7 +415,7 @@ attention_tc5_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
       int g = 0, n = 0;
       if (!SPLIT_ISSUE && (int)blockIdx.x < n_items) load_q(blockIdx.x, 0);
       for (int item = blockIdx.x; !SPLIT_ISSUE && item < n_items; item += gridDim.x, ++n) {
-        const int n_tiles = item_tiles(item % nq);
+        const int n_tiles = PREFIX ? PREFIX_TILES(item) : item_tiles(item % nq);
         const bool more = item + (int)gridDim.x < n_items;
         if (QS == 2 && more) load_q(item + gridDim.x, n + 1);            // next item's Q, one item ahead
         for (int j = 0; j < n_tiles; ++j, ++g) load_kv(item, j, g);
@@ -486,9 +508,10 @@ attention_tc5_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
     float pend_l = 1.f;
     for (int item = blockIdx.x; item < n_items; item += gridDim.x, ++n) {
       const int qt = item % nq;
-      const int n_tiles = item_tiles(qt);
+      const int n_tiles = PREFIX ? PREFIX_TILES(item) : item_tiles(qt);
       const int row = qt * BQ + rl;
       const int kmax = (row < p.ctx_rows) ? p.ctx_keys : S;
+      const int hole0 = PREFIX ? PREFIX_HOLE(item) : 0;                  // PREFIX: keys [hole0, kc) are hidden
       float m_run = -INFINITY, l_part = 0.f;
       for (int j = 0; j < n_tiles; ++j, ++g) {
         mbar_wait(s_full(SB(g)), SPH(g));
@@ -496,11 +519,11 @@ attention_tc5_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
         uint32_t r0[32];
         tmem_ld32(s_tmem0 + 64 * SB(g) + 32 * half + lane_addr, r0);
         tmem_ld_wait();
-        const int k0 = j * BKV + 32 * half;
-        if (k0 + 32 > kmax) {                                             // tile straddles this row's key limit
+        const int k0 = (PREFIX ? prefix_key0(j, hole0, p.kc) : j * BKV) + 32 * half;
+        if (k0 + 32 > kmax || (PREFIX && k0 + 32 > hole0 && k0 < p.kc)) {  // tile straddles this row's key limit (or the hole)
 #pragma unroll
           for (int i = 0; i < 32; ++i)
-            if (k0 + i >= kmax) r0[i] = 0xff800000u;                      // -inf
+            if (k0 + i >= kmax || (PREFIX && k0 + i >= hole0 && k0 + i < p.kc)) r0[i] = 0xff800000u;   // -inf
         }
         float mx;
         {
@@ -575,6 +598,8 @@ attention_tc5_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
     }
     if (pend_item >= 0) epilogue(pend_item, n - 1, pend_g, pend_l);
   }
+#undef PREFIX_TILES
+#undef PREFIX_HOLE
   tc_fence_before();
   __syncthreads();
   if (warp == 2) {
@@ -589,8 +614,9 @@ bool g_attr_dev[64];       // cudaFuncSetAttribute is per device: one handle per
 }  // namespace
 
 int launch_attention_tc5(const __nv_bfloat16* qkv16, int B, int S, int H, int ctx_rows, int ctx_keys, const AttnOut& out,
-                         cudaStream_t s, int fp16, const __nv_bfloat16* qkv_lo) {
+                         cudaStream_t s, int fp16, const __nv_bfloat16* qkv_lo, const int32_t* n_ctx, int kc) {
   STK_CHECK(qkv16 && B > 0 && S > 0 && H > 0, -1, "attention_tc5: bad arguments");
+  STK_CHECK(!n_ctx || (kc > 0 && kc < S && (ctx_keys == 0 || ctx_keys == kc)), -1, "attention_tc5: bad context-prefix window");
   STK_CHECK(out.ld % 8 == 0, -1, "attention_tc5: output pitch must be a multiple of 8");
   STK_CHECK(ctx_keys <= S && ctx_rows <= S && ctx_keys >= 0 && ctx_rows >= 0, -1, "attention_tc5: context limits exceed the sequence");
   STK_CHECK(!(fp16 && qkv_lo), -1, "attention_tc5: the split mode uses bf16 planes");
@@ -600,9 +626,12 @@ int launch_attention_tc5(const __nv_bfloat16* qkv16, int B, int S, int H, int ct
   STK_CHECK(dev >= 0 && dev < 64, -1, "attention_tc5: device ordinal out of range");
   if (!g_attr_dev[dev]) {
     STK_CUDA(cudaDeviceGetAttribute(&g_num_sms_dev[dev], cudaDevAttrMultiProcessorCount, dev));
-    STK_CUDA(cudaFuncSetAttribute(attention_tc5_kernel<true, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, A5<1>::SMEM_BYTES));
-    STK_CUDA(cudaFuncSetAttribute(attention_tc5_kernel<false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, A5<1>::SMEM_BYTES));
-    STK_CUDA(cudaFuncSetAttribute(attention_tc5_kernel<false, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, A5<3>::SMEM_BYTES));
+    STK_CUDA(cudaFuncSetAttribute(attention_tc5_kernel<true, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, A5<1>::SMEM_BYTES));
+    STK_CUDA(cudaFuncSetAttribute(attention_tc5_kernel<false, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, A5<1>::SMEM_BYTES));
+    STK_CUDA(cudaFuncSetAttribute(attention_tc5_kernel<false, 3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, A5<3>::SMEM_BYTES));
+    STK_CUDA(cudaFuncSetAttribute(attention_tc5_kernel<true, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, A5<1>::SMEM_BYTES));
+    STK_CUDA(cudaFuncSetAttribute(attention_tc5_kernel<false, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, A5<1>::SMEM_BYTES));
+    STK_CUDA(cudaFuncSetAttribute(attention_tc5_kernel<false, 3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, A5<3>::SMEM_BYTES));
     g_attr_dev[dev] = true;
   }
   const int g_num_sms = g_num_sms_dev[dev];
@@ -615,18 +644,25 @@ int launch_attention_tc5(const __nv_bfloat16* qkv16, int B, int S, int H, int ct
     STK_TRY(make_tensor_map_2d(&mql, qkv_lo, rows, cols, BQ, HD, 0));
     STK_TRY(make_tensor_map_2d(&mkvl, qkv_lo, rows, cols, BKV, HD, 0));
   }
-  Attn5Params p{out, B, S, H, ctx_rows, ctx_keys, fp16, 0.125f * 1.4426950408889634f};
+  Attn5Params p{out, B, S, H, ctx_rows, ctx_keys, fp16, 0.125f * 1.4426950408889634f, n_ctx, kc};
   const int n_items = ((S + BQ - 1) / BQ) * H * B;
   if (qkv_lo) {
     dim3 grid(std::min(n_items, A5<3>::MIN_CTAS * g_num_sms));
-    attention_tc5_kernel<false, 3><<<grid, NUM_THREADS, A5<3>::SMEM_BYTES, s>>>(mq, mkv, mql, mkvl, p);
+    if (n_ctx) attention_tc5_kernel<false, 3, true><<<grid, NUM_THREADS, A5<3>::SMEM_BYTES, s>>>(mq, mkv, mql, mkvl, p);
+    else attention_tc5_kernel<false, 3, false><<<grid, NUM_THREADS, A5<3>::SMEM_BYTES, s>>>(mq, mkv, mql, mkvl, p);
   } else {
     // persistent: two CTAs per SM walk the item list.  SELFTOK_ATTN5_CTAS_PER_SM=1 is a measurement knob (how much a CTA is
     // slowed by its co-resident twin: profiles/r2_attention_investigation.md); it never changes results.
     static const int ctas_per_sm = [] { const char* e = getenv("SELFTOK_ATTN5_CTAS_PER_SM"); return (e && e[0] == '1') ? 1 : 2; }();
     dim3 grid(std::min(n_items, ctas_per_sm * g_num_sms));
-    if (fp16) attention_tc5_kernel<true, 1><<<grid, NUM_THREADS, A5<1>::SMEM_BYTES, s>>>(mq, mkv, mql, mkvl, p);
-    else attention_tc5_kernel<false, 1><<<grid, NUM_THREADS, A5<1>::SMEM_BYTES, s>>>(mq, mkv, mql, mkvl, p);
+    if (n_ctx) {
+      if (fp16) attention_tc5_kernel<true, 1, true><<<grid, NUM_THREADS, A5<1>::SMEM_BYTES, s>>>(mq, mkv, mql, mkvl, p);
+      else attention_tc5_kernel<false, 1, true><<<grid, NUM_THREADS, A5<1>::SMEM_BYTES, s>>>(mq, mkv, mql, mkvl, p);
+    } else if (fp16) {
+      attention_tc5_kernel<true, 1, false><<<grid, NUM_THREADS, A5<1>::SMEM_BYTES, s>>>(mq, mkv, mql, mkvl, p);
+    } else {
+      attention_tc5_kernel<false, 1, false><<<grid, NUM_THREADS, A5<1>::SMEM_BYTES, s>>>(mq, mkv, mql, mkvl, p);
+    }
   }
   count_launch();
   STK_CUDA(cudaGetLastError());

@@ -108,6 +108,13 @@ struct selftok_engine {
   size_t user_ws_bytes[2] = {0, 0};
   std::map<std::pair<int, int>, std::pair<cudaGraphExec_t, int64_t>> graphs;   // (B, steps) -> (exec, launches)
   std::map<int, std::pair<cudaGraphExec_t, int64_t>> enc_graphs;               // encode, B -> (exec, launches)
+  // decode from a token prefix: per-image visible-token counts at a fixed device address (captured graphs read it), and the
+  // graphs keyed by (B, steps, per-step context rows), least recently used dropped beyond kPrefixGraphs
+  int32_t* n_dev = nullptr;
+  int n_cap = 0;
+  struct PrefixGraph { cudaGraphExec_t exec; int64_t launches; uint64_t used; };
+  std::map<std::vector<int>, PrefixGraph> prefix_graphs;
+  uint64_t prefix_tick = 0;
   int64_t last_launches = 0;
   // optional per-kernel-class timing (CUDA events around every launch; only meaningful with graphs disabled)
   bool prof_on = false;
@@ -260,6 +267,14 @@ extern "C" __attribute__((visibility("default"))) int selftok_create(const selft
   return SELFTOK_OK;
 }
 
+static const size_t kPrefixGraphs = 4;
+// captured decode graphs hold pointers into the decode workspace and the prefix-count buffer
+static void drop_decode_graphs(selftok_engine* e) {
+  for (auto& g : e->graphs) cudaGraphExecDestroy(g.second.first);
+  e->graphs.clear();
+  for (auto& g : e->prefix_graphs) cudaGraphExecDestroy(g.second.exec);
+  e->prefix_graphs.clear();
+}
 static void free_dws(selftok_engine* e) {
   if (e->dws.own) { cudaFree(e->dws.own); e->bytes -= (int64_t)e->dws.own_bytes; }
   e->dws = DecodeWs();
@@ -275,7 +290,8 @@ extern "C" __attribute__((visibility("default"))) int selftok_destroy(selftok_ha
   if (!e) return SELFTOK_OK;
   cudaSetDevice(e->cfg.device);
   cudaDeviceSynchronize();
-  for (auto& g : e->graphs) cudaGraphExecDestroy(g.second.first);
+  drop_decode_graphs(e);
+  if (e->n_dev) cudaFree(e->n_dev);
   for (auto& kv : e->w) cudaFree(kv.second.d);
   free_pool(e, e->allocs);
   if (e->bad_ids) cudaFree(e->bad_ids);
@@ -840,10 +856,16 @@ extern "C" __attribute__((visibility("default"))) int selftok_vq_argmax(selftok_
   return SELFTOK_OK;
 }
 
-static int run_lookup(selftok_engine* e, const int64_t* tokens, int B, float* outs_q, cudaStream_t s) {
+// n_tok (device [B], optional): image b from its first n_tok[b] tokens
+static int run_lookup(selftok_engine* e, const int64_t* tokens, int B, float* outs_q, cudaStream_t s, const int32_t* n_tok = nullptr) {
   GETW(cb, "encoder.quantizer._codebook.embed");
   GETW(lw, "encoder.final_layer_norm3.weight");
   GETW(lb, "encoder.final_layer_norm3.bias");
+  if (n_tok) {
+    PROF(PC_OTHER, launch_lookup_ln3_prefix(tokens, B, e->cfg.K, n_tok, cb->d, e->cfg.codebook_size, e->cfg.code_dim, lw->d, lb->d,
+                                            outs_q, e->bad_ids, s));
+    return 0;
+  }
   PROF(PC_OTHER, launch_lookup_ln3(tokens, (int64_t)B * e->cfg.K, cb->d, e->cfg.codebook_size, e->cfg.code_dim, lw->d, lb->d, outs_q,
                                    e->bad_ids, s));
   return 0;
@@ -927,8 +949,7 @@ static int layout_dws(selftok_engine* e, DecodeWs& w, int64_t B, Arena& A) {
 }
 static int ensure_dws(selftok_engine* e, int B) {
   if (e->dws.B >= B) return 0;
-  for (auto& g : e->graphs) cudaGraphExecDestroy(g.second.first);   // graphs hold pointers into the old workspace
-  e->graphs.clear();
+  drop_decode_graphs(e);
   free_dws(e);
   return place_ws(e, 1, e->dws, B, [&](DecodeWs& w, int64_t b, Arena& A) { return layout_dws(e, w, b, A); });
 }
@@ -1024,8 +1045,9 @@ static int final_layer(selftok_engine* e, int B, const float* fm, float* o_out, 
 //   uncond     unconditional branch of the guided sampler (MMDiT.cfg_inference, mmdit.py:1117-1163): Kc must be 0 (no row of
 //              that pass sees a context key, so the context stream is dropped -- exact), x-stream adaLN from the integer timestep
 //   o_out      final-layer output [B*N, p*p*C]
+//   n_ctx      optional device [B]: image b sees only the context keys < min(Kc, n_ctx[b]) (decode from a token prefix)
 static int joint_blocks(selftok_engine* e, int B, int Kc, int step, bool ctx_self, cudaStream_t s, bool uncond = false,
-                        float* o_out = nullptr) {
+                        float* o_out = nullptr, const int32_t* n_ctx = nullptr) {
   const selftok_config_t& c = e->cfg;
   DecodeWs& w = e->dws;
   const int D = e->D, N = e->Nimg, L = c.dit_depth, T = e->steps, S = Kc + N;
@@ -1067,7 +1089,8 @@ static int joint_blocks(selftok_engine* e, int B, int Kc, int step, bool ctx_sel
       ao.hi_a = w.attn_c_hi; ao.lo_a = w.attn_c_lo; ao.hi_b = w.attn_x_hi; ao.lo_b = w.attn_x_lo;
       ao.fp16 = fp16;
       const int ctx_rows = ctx_self ? Kc : 0, ctx_keys = ctx_self ? Kc : 0;
-      PROF(PC_ATTN, launch_attention_tc5(w.qkv_hi, B, S, e->H, ctx_rows, ctx_keys, ao, s, fp16, nsplit(e) == 3 ? w.qkv_lo : nullptr));
+      PROF(PC_ATTN, launch_attention_tc5(w.qkv_hi, B, S, e->H, ctx_rows, ctx_keys, ao, s, fp16, nsplit(e) == 3 ? w.qkv_lo : nullptr,
+                                         n_ctx, Kc));
       // post_attention (mmdit.py:485-496); the pre_only context block of the last layer stops here
       Epilogue erx, erc;
       erx.mode = EPI_RESID; erx.out = w.x; erx.resid = w.x; erx.ldo = D; erx.gate = xmod + 2 * D; erx.gate_ld = 6 * D; erx.gate_period = 1;
@@ -1107,11 +1130,12 @@ static int joint_blocks(selftok_engine* e, int B, int Kc, int step, bool ctx_sel
     if (!tc_mode(e)) {
       ao.f32_a = w.attn_c; ao.f32_b = w.attn_x;
       PROF(PC_ATTN, launch_attention_f32(w.qkv, 3 * D, (int64_t)S * 3 * D, w.qkv + D, w.qkv + 2 * D, 3 * D, (int64_t)S * 3 * D, S,
-                                   nullptr, nullptr, 0, 0, 0, ao, B, S, e->H, 64, ctx_rows, ctx_keys, s));
+                                   nullptr, nullptr, 0, 0, 0, ao, B, S, e->H, 64, ctx_rows, ctx_keys, s, n_ctx, Kc));
     } else {
       ao.hi_a = w.attn_c_hi; ao.lo_a = w.attn_c_lo; ao.hi_b = w.attn_x_hi; ao.lo_b = w.attn_x_lo;
       ao.fp16 = is_fp16(e);
-      PROF(PC_ATTN, launch_attention_tc5(w.qkv_hi, B, S, e->H, ctx_rows, ctx_keys, ao, s, is_fp16(e), nsplit(e) == 3 ? w.qkv_lo : nullptr));
+      PROF(PC_ATTN, launch_attention_tc5(w.qkv_hi, B, S, e->H, ctx_rows, ctx_keys, ao, s, is_fp16(e), nsplit(e) == 3 ? w.qkv_lo : nullptr,
+                                         n_ctx, Kc));
     }
     if (ctx_post)
       STK_TRY(post_attention(e, pc, w.ctx, Mc, cmod, 6 * D, Kc, w.attn_c, w.attn_c_hi, w.attn_c_lo, w.a_c, w.a_c_hi, w.a_c_lo,
@@ -1133,48 +1157,61 @@ static int context_embed(selftok_engine* e, int B, cudaStream_t s) {
   return lin32(e, "model.context_embedder", w.outs_q, e->cfg.code_dim, (int64_t)B * e->cfg.K, ep, s);
 }
 
+// Context rows of schedule row `step`: the visible prefix k + 1 (rows beyond it are masked everywhere and dropped -- exact),
+// capped at n_max, the longest token prefix of the batch (decode from a token prefix, the same truncation with min(k + 1, n))
+static int ctx_rows_at(const selftok_engine* e, int step, int n_max) {
+  return (e->k[step] < n_max - 1 ? e->k[step] : n_max - 1) + 1;
+}
+
+// Per-image token prefixes of one call: device counts [B] (engine-owned buffer) and their maximum; n == NULL: every K token
+struct Prefix {
+  const int32_t* n = nullptr;
+  int n_max = 0;
+};
+
 // One MMDiT.forward (mmdit.py:992-1101) at schedule row `step` on ws.x_lat; leaves the patch outputs in ws.o_final.
-static int dit_forward(selftok_engine* e, int B, int step, cudaStream_t s) {
+static int dit_forward(selftok_engine* e, int B, int step, cudaStream_t s, Prefix pre = Prefix()) {
   const selftok_config_t& c = e->cfg;
   DecodeWs& w = e->dws;
-  const int D = e->D, Kc = e->k[step] + 1;
+  const int D = e->D, Kc = pre.n ? ctx_rows_at(e, step, pre.n_max) : e->k[step] + 1;
   PROF(PC_OTHER, launch_patchify(w.x_lat, w.patch, B, c.in_channels, c.latent, c.latent, c.dit_patch, s));
   STK_TRY(x_embed(e, B, s));
   PROF(PC_OTHER, launch_copy_rows(w.ctx0, (int64_t)c.K * D, w.ctx, (int64_t)Kc * D, B, (int64_t)Kc * D, s));
   // context rows see the image keys unless the handle was created with context_see_xt = 0 (sd3/mmdit.py:1012,1060; the
   // reference pipeline's sampler passes context_see_xt=True, SelftokPipeline.py:259)
-  return joint_blocks(e, B, Kc, step, /*ctx_self=*/e->cfg.context_see_xt == 0, s);
+  return joint_blocks(e, B, Kc, step, /*ctx_self=*/e->cfg.context_see_xt == 0, s, false, nullptr, pre.n);
 }
 
 // The two evaluations of one guided step (sample_one_step with cfg_scale != 1, rectified_flow.py:280-289): the conditional
 // one -- called there WITHOUT context_see_xt, i.e. context rows only see the visible context keys -- into ws.o_final, and
 // MMDiT.cfg_inference (context = zeros, every context key masked for every row: the image stream alone, integer timestep)
 // into ws.o_final_u.
-static int dit_forward_cfg(selftok_engine* e, int B, int step, cudaStream_t s) {
+static int dit_forward_cfg(selftok_engine* e, int B, int step, cudaStream_t s, Prefix pre = Prefix()) {
   const selftok_config_t& c = e->cfg;
   DecodeWs& w = e->dws;
-  const int D = e->D, Kc = e->k[step] + 1;
+  const int D = e->D, Kc = pre.n ? ctx_rows_at(e, step, pre.n_max) : e->k[step] + 1;
   STK_CHECK(e->has_cfg, SELFTOK_ERR_STATE, "guided sampling needs selftok_set_cfg_schedule before selftok_finalize");
   PROF(PC_OTHER, launch_patchify(w.x_lat, w.patch, B, c.in_channels, c.latent, c.latent, c.dit_patch, s));
   STK_TRY(x_embed(e, B, s));
   PROF(PC_OTHER, launch_copy_rows(w.ctx0, (int64_t)c.K * D, w.ctx, (int64_t)Kc * D, B, (int64_t)Kc * D, s));
-  STK_TRY(joint_blocks(e, B, Kc, step, /*ctx_self=*/true, s, /*uncond=*/false, w.o_final));
+  STK_TRY(joint_blocks(e, B, Kc, step, /*ctx_self=*/true, s, /*uncond=*/false, w.o_final, pre.n));
   STK_TRY(x_embed(e, B, s));
   return joint_blocks(e, B, 0, step, /*ctx_self=*/false, s, /*uncond=*/true, w.o_final_u);
 }
 
-static int decode_body(selftok_engine* e, int B, int steps, cudaStream_t s, bool guided = false, float cfg_scale = 1.f) {
+static int decode_body(selftok_engine* e, int B, int steps, cudaStream_t s, bool guided = false, float cfg_scale = 1.f,
+                       Prefix pre = Prefix()) {
   const selftok_config_t& c = e->cfg;
   DecodeWs& w = e->dws;
-  STK_TRY(run_lookup(e, w.tokens, B, w.outs_q, s));
+  STK_TRY(run_lookup(e, w.tokens, B, w.outs_q, s, pre.n));
   STK_TRY(context_embed(e, B, s));
   for (int i = 0; i < steps; ++i) {
     // euler_step (rectified_flow.py:301-303): x <- x - (t_i - t_{i+1}) * v, fused with unpatchify
     if (!guided) {
-      STK_TRY(dit_forward(e, B, i, s));
+      STK_TRY(dit_forward(e, B, i, s, pre));
       PROF(PC_OTHER, launch_unpatchify_axpy(w.o_final, w.x_lat, w.x_lat, e->dt[i], B, c.in_channels, c.latent / c.dit_patch, c.dit_patch, s));
     } else {
-      STK_TRY(dit_forward_cfg(e, B, i, s));
+      STK_TRY(dit_forward_cfg(e, B, i, s, pre));
       PROF(PC_OTHER, launch_unpatchify_axpy(w.o_final, w.x_lat, w.x_lat, e->dt[i], B, c.in_channels, c.latent / c.dit_patch, c.dit_patch, s,
                                             w.o_final_u, cfg_scale));
     }
@@ -1203,8 +1240,7 @@ extern "C" __attribute__((visibility("default"))) int selftok_set_workspace(self
   e->user_ws_bytes[op] = ws_dev ? bytes : 0;
   if (op == 0) free_ews(e);
   else {
-    for (auto& g : e->graphs) cudaGraphExecDestroy(g.second.first);
-    e->graphs.clear();
+    drop_decode_graphs(e);
     free_dws(e);
   }
   return SELFTOK_OK;
@@ -1217,7 +1253,32 @@ extern "C" __attribute__((visibility("default"))) int selftok_set_use_graph(self
 }
 
 static int decode_impl(selftok_handle_t e, const int64_t* tokens_dev, const float* noise_dev, int B, int steps, float* x0_out_dev,
-                       void* stream, bool guided, float cfg_scale);
+                       void* stream, bool guided, float cfg_scale, const int32_t* n_host = nullptr);
+
+// Per-image token prefixes from the host: every n_b in [1, K] (checked before anything is launched), copied into the
+// engine-owned device buffer on `s` -- after the copy the caller's array is not read again
+static int check_prefix(selftok_engine* e, const int32_t* n_host, int B, int* n_max) {
+  STK_CHECK(n_host, SELFTOK_ERR_BAD_ARG, "token prefix: null n_tokens");
+  *n_max = 0;
+  for (int b = 0; b < B; ++b) {
+    STK_CHECK(n_host[b] >= 1 && n_host[b] <= e->cfg.K, SELFTOK_ERR_BAD_ARG,
+              "token prefix: n_tokens[" + std::to_string(b) + "] = " + std::to_string(n_host[b]) + " is outside [1, K]");
+    if (n_host[b] > *n_max) *n_max = n_host[b];
+  }
+  return 0;
+}
+static int load_prefix(selftok_engine* e, const int32_t* n_host, int B, int n_max, cudaStream_t s, Prefix* pre) {
+  if (e->n_cap < B) {
+    drop_decode_graphs(e);
+    if (e->n_dev) { cudaFree(e->n_dev); e->n_dev = nullptr; e->n_cap = 0; }
+    STK_CUDA(cudaMalloc(&e->n_dev, sizeof(int32_t) * B));
+    e->n_cap = B;
+  }
+  STK_CUDA(cudaMemcpyAsync(e->n_dev, n_host, sizeof(int32_t) * B, cudaMemcpyHostToDevice, s));
+  pre->n = e->n_dev;
+  pre->n_max = n_max;
+  return 0;
+}
 
 extern "C" __attribute__((visibility("default"))) int selftok_decode(selftok_handle_t e, const int64_t* tokens_dev, const float* noise_dev, int B, int steps,
                               float* x0_out_dev, void* stream) {
@@ -1231,14 +1292,28 @@ extern "C" __attribute__((visibility("default"))) int selftok_decode_cfg(selftok
   return decode_impl(e, tokens_dev, noise_dev, B, steps, x0_out_dev, stream, true, cfg_scale);
 }
 
+// Decode from a token prefix: image b from its first n_tokens_host[b] tokens (super_mask of p_sample_loop, rectified_flow.py:
+// 182,227-228).  cfg_scale == 1: the plain sampler (captured graph); otherwise the guided sampler (eager), the prefix applied
+// to its conditional evaluation.
+extern "C" __attribute__((visibility("default"))) int selftok_decode_prefix(selftok_handle_t e, const int64_t* tokens_dev, const int32_t* n_tokens_host,
+                                                                       const float* noise_dev, int B, int steps, float cfg_scale,
+                                                                       float* x0_out_dev, void* stream) {
+  STK_CHECK(n_tokens_host, SELFTOK_ERR_BAD_ARG, "selftok_decode_prefix: null n_tokens");
+  return decode_impl(e, tokens_dev, noise_dev, B, steps, x0_out_dev, stream, cfg_scale != 1.f, cfg_scale, n_tokens_host);
+}
+
 static int decode_impl(selftok_handle_t e, const int64_t* tokens_dev, const float* noise_dev, int B, int steps, float* x0_out_dev,
-                       void* stream, bool guided, float cfg_scale) {
+                       void* stream, bool guided, float cfg_scale, const int32_t* n_host) {
   HOT_PROLOGUE(e);
   STK_CHECK(!guided || e->has_cfg, SELFTOK_ERR_STATE, "selftok_decode_cfg: selftok_set_cfg_schedule was not called before finalize");
   STK_CHECK(tokens_dev && noise_dev && x0_out_dev && B > 0, SELFTOK_ERR_BAD_ARG, "selftok_decode: bad argument");
   STK_CHECK(!e->cfg.renderer, SELFTOK_ERR_STATE, "handle was created for the renderer; use selftok_render");
   STK_CHECK(steps > 0 && steps <= e->steps, SELFTOK_ERR_BAD_ARG, "steps exceeds the schedule");
+  int n_max = 0;
+  if (n_host) STK_TRY(check_prefix(e, n_host, B, &n_max));
   STK_TRY(ensure_dws(e, B));
+  Prefix pre;
+  if (n_host) STK_TRY(load_prefix(e, n_host, B, n_max, s, &pre));
   DecodeWs& w = e->dws;
   const int64_t nlat = (int64_t)B * e->cfg.in_channels * e->cfg.latent * e->cfg.latent;
   if (tokens_dev != w.tokens) STK_CUDA(cudaMemcpyAsync(w.tokens, tokens_dev, sizeof(int64_t) * B * e->cfg.K, cudaMemcpyDeviceToDevice, s));
@@ -1246,8 +1321,46 @@ static int decode_impl(selftok_handle_t e, const int64_t* tokens_dev, const floa
   // eager when asked to, for the guided loop (cfg_scale is a kernel argument) and whenever per-launch profiling is on (events
   // recorded inside a capture never execute on a real stream: their elapsed times would be garbage)
   if (!e->use_graph || guided || e->prof_on) {
-    STK_TRY(decode_body(e, B, steps, s, guided, cfg_scale));
+    STK_TRY(decode_body(e, B, steps, s, guided, cfg_scale, pre));
     e->last_launches = g_launch_count - launches0;
+  } else if (pre.n) {
+    // one graph per (B, steps, context rows of every step); the counts it reads were refreshed above, on the same stream
+    std::vector<int> key = {B, steps};
+    for (int i = 0; i < steps; ++i) key.push_back(ctx_rows_at(e, i, pre.n_max));
+    auto it = e->prefix_graphs.find(key);
+    if (it == e->prefix_graphs.end()) {
+      if (e->prefix_graphs.size() >= kPrefixGraphs) {
+        auto lru = e->prefix_graphs.begin();
+        for (auto j = e->prefix_graphs.begin(); j != e->prefix_graphs.end(); ++j)
+          if (j->second.used < lru->second.used) lru = j;
+        STK_CUDA(cudaStreamSynchronize(s));                          // a replay of it may still be queued on this stream
+        cudaGraphExecDestroy(lru->second.exec);
+        e->prefix_graphs.erase(lru);
+      }
+      cudaStream_t cs;
+      STK_CUDA(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
+      {
+        const cudaError_t be = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
+        if (be != cudaSuccess) {
+          cudaStreamDestroy(cs);
+          STK_CUDA(be);
+        }
+      }
+      const int64_t l0 = g_launch_count;
+      int st = decode_body(e, B, steps, cs, false, 1.f, pre);
+      cudaGraph_t graph = nullptr;
+      cudaError_t ce = cudaStreamEndCapture(cs, &graph);
+      cudaStreamDestroy(cs);
+      if (st != 0) { if (graph) cudaGraphDestroy(graph); return st; }
+      STK_CUDA(ce);
+      cudaGraphExec_t exec;
+      STK_CUDA(cudaGraphInstantiate(&exec, graph, 0));
+      cudaGraphDestroy(graph);
+      it = e->prefix_graphs.emplace(key, selftok_engine::PrefixGraph{exec, g_launch_count - l0, 0}).first;
+    }
+    it->second.used = ++e->prefix_tick;
+    STK_CUDA(cudaGraphLaunch(it->second.exec, s));
+    e->last_launches = it->second.launches;
   } else {
     auto key = std::make_pair(B, steps);
     auto it = e->graphs.find(key);
@@ -1280,43 +1393,74 @@ static int decode_impl(selftok_handle_t e, const int64_t* tokens_dev, const floa
   return SELFTOK_OK;
 }
 
-extern "C" __attribute__((visibility("default"))) int selftok_dit_velocity(selftok_handle_t e, const int64_t* tokens_dev, const float* x_dev, int B, int step,
-                                    float* v_out_dev, void* stream) {
+static int velocity_impl(selftok_handle_t e, const int64_t* tokens_dev, const int32_t* n_host, const float* x_dev, int B, int step,
+                         float* v_out_dev, void* stream) {
   HOT_PROLOGUE(e);
   STK_CHECK(tokens_dev && x_dev && v_out_dev && B > 0, SELFTOK_ERR_BAD_ARG, "selftok_dit_velocity: bad argument");
   STK_CHECK(!e->cfg.renderer, SELFTOK_ERR_STATE, "renderer handle");
   STK_CHECK(step >= 0 && step < e->steps, SELFTOK_ERR_BAD_ARG, "step out of range");
+  int n_max = 0;
+  if (n_host) STK_TRY(check_prefix(e, n_host, B, &n_max));
   STK_TRY(ensure_dws(e, B));
+  Prefix pre;
+  if (n_host) STK_TRY(load_prefix(e, n_host, B, n_max, s, &pre));
   DecodeWs& w = e->dws;
   const selftok_config_t& c = e->cfg;
   const int64_t nlat = (int64_t)B * c.in_channels * c.latent * c.latent;
   STK_CUDA(cudaMemcpyAsync(w.tokens, tokens_dev, sizeof(int64_t) * B * c.K, cudaMemcpyDeviceToDevice, s));
   STK_CUDA(cudaMemcpyAsync(w.x_lat, x_dev, sizeof(float) * nlat, cudaMemcpyDeviceToDevice, s));
-  STK_TRY(run_lookup(e, w.tokens, B, w.outs_q, s));
+  STK_TRY(run_lookup(e, w.tokens, B, w.outs_q, s, pre.n));
   STK_TRY(context_embed(e, B, s));
-  STK_TRY(dit_forward(e, B, step, s));
+  STK_TRY(dit_forward(e, B, step, s, pre));
   PROF(PC_OTHER, launch_unpatchify_axpy(w.o_final, nullptr, v_out_dev, -1.f, B, c.in_channels, c.latent / c.dit_patch, c.dit_patch, s));
   e->last_launches = g_launch_count - launches0;
   return SELFTOK_OK;
 }
 
-extern "C" __attribute__((visibility("default"))) int selftok_render(selftok_handle_t e, const int64_t* tokens_dev, int B, float* x0_out_dev, void* stream) {
+extern "C" __attribute__((visibility("default"))) int selftok_dit_velocity(selftok_handle_t e, const int64_t* tokens_dev, const float* x_dev, int B, int step,
+                                    float* v_out_dev, void* stream) {
+  return velocity_impl(e, tokens_dev, nullptr, x_dev, B, step, v_out_dev, stream);
+}
+
+extern "C" __attribute__((visibility("default"))) int selftok_dit_velocity_prefix(selftok_handle_t e, const int64_t* tokens_dev, const int32_t* n_tokens_host,
+                                                                             const float* x_dev, int B, int step, float* v_out_dev, void* stream) {
+  STK_CHECK(n_tokens_host, SELFTOK_ERR_BAD_ARG, "selftok_dit_velocity_prefix: null n_tokens");
+  return velocity_impl(e, tokens_dev, n_tokens_host, x_dev, B, step, v_out_dev, stream);
+}
+
+static int render_impl(selftok_handle_t e, const int64_t* tokens_dev, const int32_t* n_host, int B, float* x0_out_dev, void* stream) {
   HOT_PROLOGUE(e);
   STK_CHECK(tokens_dev && x0_out_dev && B > 0, SELFTOK_ERR_BAD_ARG, "selftok_render: bad argument");
   STK_CHECK(e->cfg.renderer, SELFTOK_ERR_STATE, "handle was not created for the renderer");
+  int n_max = 0;
+  if (n_host) STK_TRY(check_prefix(e, n_host, B, &n_max));
   STK_TRY(ensure_dws(e, B));
+  Prefix pre;
+  if (n_host) STK_TRY(load_prefix(e, n_host, B, n_max, s, &pre));
   DecodeWs& w = e->dws;
   const selftok_config_t& c = e->cfg;
+  // context rows: all K, or the batch's longest prefix (image b then masks the context keys [n_b, n_max))
+  const int Kc = pre.n ? pre.n_max : c.K;
   if (tokens_dev != w.tokens) STK_CUDA(cudaMemcpyAsync(w.tokens, tokens_dev, sizeof(int64_t) * B * c.K, cudaMemcpyDeviceToDevice, s));
-  STK_TRY(run_lookup(e, w.tokens, B, w.outs_q, s));
+  STK_TRY(run_lookup(e, w.tokens, B, w.outs_q, s, pre.n));
   STK_TRY(context_embed(e, B, s));
-  // x = mask_token + positional_embedding (mmdit.py:1518-1522); context = full K rows, context rows see context only
+  // x = mask_token + positional_embedding (mmdit.py:1518-1522); context rows see context only
   PROF(PC_OTHER, launch_bcast_rows(e->rend_x0, nullptr, w.x, B, e->Nimg, e->D, s));
-  PROF(PC_OTHER, launch_copy_rows(w.ctx0, (int64_t)c.K * e->D, w.ctx, (int64_t)c.K * e->D, B, (int64_t)c.K * e->D, s));
-  STK_TRY(joint_blocks(e, B, c.K, 0, /*ctx_self=*/true, s));
+  PROF(PC_OTHER, launch_copy_rows(w.ctx0, (int64_t)c.K * e->D, w.ctx, (int64_t)Kc * e->D, B, (int64_t)Kc * e->D, s));
+  STK_TRY(joint_blocks(e, B, Kc, 0, /*ctx_self=*/true, s, false, nullptr, pre.n));
   PROF(PC_OTHER, launch_unpatchify_axpy(w.o_final, nullptr, x0_out_dev, -1.f, B, c.in_channels, c.latent / c.dit_patch, c.dit_patch, s));
   e->last_launches = g_launch_count - launches0;
   return SELFTOK_OK;
+}
+
+extern "C" __attribute__((visibility("default"))) int selftok_render(selftok_handle_t e, const int64_t* tokens_dev, int B, float* x0_out_dev, void* stream) {
+  return render_impl(e, tokens_dev, nullptr, B, x0_out_dev, stream);
+}
+
+extern "C" __attribute__((visibility("default"))) int selftok_render_prefix(selftok_handle_t e, const int64_t* tokens_dev, const int32_t* n_tokens_host,
+                                                                       int B, float* x0_out_dev, void* stream) {
+  STK_CHECK(n_tokens_host, SELFTOK_ERR_BAD_ARG, "selftok_render_prefix: null n_tokens");
+  return render_impl(e, tokens_dev, n_tokens_host, B, x0_out_dev, stream);
 }
 
 // ------------------------------------------------------------------------------------------------ host-buffer variants

@@ -65,10 +65,11 @@ struct AttnOut {
 };
 // softmax(q k^T / sqrt(hd)) v in fp32.  q rows: q + b*q_bs + s*q_ld + h*hd; keys = segment 1 (S1 rows) followed by
 // segment 2 (S2 rows).  Rows < ctx_rows only see keys < ctx_keys (renderer rule); ctx_rows = 0 -> dense.
+// n_ctx != NULL: the context-prefix window of launch_attention_tc5 over the key index (kc = context keys).
 int launch_attention_f32(const float* q, int64_t q_ld, int64_t q_bs, const float* k1, const float* v1, int64_t kv1_ld,
                          int64_t kv1_bs, int S1, const float* k2, const float* v2, int64_t kv2_ld, int64_t kv2_bs,
                          int S2, const AttnOut& out, int B, int Sq, int H, int hd, int ctx_rows, int ctx_keys,
-                         cudaStream_t s);
+                         cudaStream_t s, const int32_t* n_ctx = nullptr, int kc = 0);
 // Fused VQ: project_in + l2norm + argmax over the codebook + gather + final_layer_norm3.
 int launch_vq(const float* z, int64_t R, int Q, const float* w_in, const float* b_in, const float* codebook,
               const float* codebook_t, int n_codes, int code_dim, const float* ln_w, const float* ln_b,
@@ -76,6 +77,10 @@ int launch_vq(const float* z, int64_t R, int Q, const float* w_in, const float* 
 // ids outside [0, n_codes): row poisoned with NaN and counted in *bad_ids (may be NULL)
 int launch_lookup_ln3(const int64_t* ids, int64_t R, const float* codebook, int n_codes, int code_dim,
                       const float* ln_w, const float* ln_b, float* outs_q, int* bad_ids, cudaStream_t s);
+// the same over B images of K ids, image b from its first n_tok[b] ids only (device array [B]): later positions get zero
+// rows and their ids are never read
+int launch_lookup_ln3_prefix(const int64_t* ids, int B, int K, const int32_t* n_tok, const float* codebook, int n_codes,
+                             int code_dim, const float* ln_w, const float* ln_b, float* outs_q, int* bad_ids, cudaStream_t s);
 // [B,C,Hh,Ww] latents -> [B*(Hh/p)*(Ww/p), C*p*p] patch rows ((c,ph,pw) fastest-last, Conv2d weight order)
 int launch_patchify(const float* x, float* out, int B, int C, int Hh, int Ww, int p, cudaStream_t s);
 // x_lat[b,c,h*p+ph,w*p+pw] = x_in[...] - dt * o[b, h*g+w, (ph*p+pw)*C + c]   (unpatchify + Euler; dt = -1 & x_in NULL: plain unpatchify)
@@ -114,7 +119,10 @@ void gemm_tc_set_ctas(int n);   // 2 (default): cta_group::2 pair kernel; 1: sin
 // qkv planes: packed 16-bit [B,S,3,H,64] (hi, and lo for the split mode), written by the QKV GEMM epilogue
 // tcgen05 / TMEM attention (attn_tc5.cu): single-pass 16-bit operands (fp16 != 0: IEEE half, else bf16), or -- with the lo
 // planes given -- the fp32-faithful split-bf16 mode (three MMAs per product, P split in registers)
+// n_ctx != NULL (decode from a token prefix): image b additionally ignores the context keys [min(kc, n_ctx[b]), kc), kc = the
+// context rows of the joint sequence (ctx_keys must be 0 or kc); n_ctx is a device array [B], every entry >= 1
 int launch_attention_tc5(const __nv_bfloat16* qkv16, int B, int S, int H, int ctx_rows, int ctx_keys, const AttnOut& out,
-                         cudaStream_t s, int fp16, const __nv_bfloat16* qkv_lo = nullptr);
+                         cudaStream_t s, int fp16, const __nv_bfloat16* qkv_lo = nullptr, const int32_t* n_ctx = nullptr,
+                         int kc = 0);
 
 }  // namespace stk

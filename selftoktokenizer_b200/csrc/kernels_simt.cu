@@ -461,9 +461,11 @@ struct AttnParams {
   AttnOut out;
   int Sq, H, ctx_rows, ctx_keys;
   float scale;
+  const int32_t* n_ctx;   // PREFIX: visible context tokens per image [B]
+  int kc;                 // PREFIX: context keys; image b ignores keys [min(kc, n_ctx[b]), kc)
 };
 
-template <int HD>
+template <int HD, bool PREFIX = false>
 __global__ void __launch_bounds__(256) attention_f32_kernel(const AttnParams p) {
   constexpr int BQ = 64, BKV = 64, DV = HD / 16;
   extern __shared__ __align__(16) float smem[];
@@ -494,7 +496,9 @@ __global__ void __launch_bounds__(256) attention_f32_kernel(const AttnParams p) 
 #pragma unroll
   for (int i = 0; i < 4; ++i) kmax_row[i] = (q0 + ty * 4 + i < p.ctx_rows) ? p.ctx_keys : Sk;
   int kmax_cta = (q0 + BQ <= p.ctx_rows) ? p.ctx_keys : Sk;        // all rows of this CTA are context rows
+  const int hole0 = PREFIX ? min(p.kc, p.n_ctx[b]) : 0;            // PREFIX: keys [hole0, kc) are hidden
   for (int k0 = 0; k0 < kmax_cta; k0 += BKV) {
+    if (PREFIX && k0 >= hole0 && k0 + BKV <= p.kc) continue;      // tile wholly inside the hole
     __syncthreads();                                              // previous tile fully consumed (also covers Qt)
     for (int f = tid; f < BKV * HD / 4; f += 256) {
       int r = f / (HD / 4), d4 = (f % (HD / 4)) * 4;
@@ -553,7 +557,7 @@ __global__ void __launch_bounds__(256) attention_f32_kernel(const AttnParams p) 
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
         int key = k0 + tx * 4 + j;
-        if (key >= kmax_row[i]) sacc[i][j] = -INFINITY;
+        if (key >= kmax_row[i] || (PREFIX && key >= hole0 && key < p.kc)) sacc[i][j] = -INFINITY;
         mx = fmaxf(mx, sacc[i][j]);
       }
 #pragma unroll
@@ -652,12 +656,14 @@ __global__ void __launch_bounds__(256) attention_f32_kernel(const AttnParams p) 
 int launch_attention_f32(const float* q, int64_t q_ld, int64_t q_bs, const float* k1, const float* v1, int64_t kv1_ld,
                          int64_t kv1_bs, int S1, const float* k2, const float* v2, int64_t kv2_ld, int64_t kv2_bs,
                          int S2, const AttnOut& out, int B, int Sq, int H, int hd, int ctx_rows, int ctx_keys,
-                         cudaStream_t s) {
+                         cudaStream_t s, const int32_t* n_ctx, int kc) {
   STK_CHECK(q && k1 && v1 && B > 0 && Sq > 0 && H > 0 && S1 > 0 && S2 >= 0, -1, "attention_f32: bad arguments");
+  STK_CHECK(!n_ctx || (hd == 64 && kc > 0 && kc < S1 + S2 && (ctx_keys == 0 || ctx_keys == kc)), -1,
+            "attention_f32: bad context-prefix window");
   STK_CHECK(hd == 16 || hd == 32 || hd == 64, -2, "attention_f32: head_dim must be 16, 32 or 64");
   STK_CHECK(q_ld % 4 == 0 && kv1_ld % 4 == 0 && (S2 == 0 || kv2_ld % 4 == 0), -1, "attention_f32: strides must be multiples of 4");
   AttnParams p{q, q_ld, q_bs, k1, v1, kv1_ld, kv1_bs, S1, k2, v2, kv2_ld, kv2_bs, S2, out, Sq, H, ctx_rows, ctx_keys,
-               1.0f / sqrtf((float)hd)};
+               1.0f / sqrtf((float)hd), n_ctx, kc};
   dim3 grid((Sq + 63) / 64, H, B);
   size_t smem = sizeof(float) * (size_t)(hd * 68 * 2 + 64 * hd + 64 * 68);
   if (hd == 64) {
@@ -666,9 +672,11 @@ int launch_attention_f32(const float* q, int64_t q_ld, int64_t q_bs, const float
     STK_CUDA(cudaGetDevice(&dev));
     if (dev >= 0 && dev < 64 && !attr[dev]) {
       STK_CUDA(cudaFuncSetAttribute(attention_f32_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      STK_CUDA(cudaFuncSetAttribute(attention_f32_kernel<64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       attr[dev] = true;
     }
-    attention_f32_kernel<64><<<grid, 256, smem, s>>>(p);
+    if (n_ctx) attention_f32_kernel<64, true><<<grid, 256, smem, s>>>(p);
+    else attention_f32_kernel<64><<<grid, 256, smem, s>>>(p);
   } else if (hd == 32) {
     attention_f32_kernel<32><<<grid, 256, smem, s>>>(p);
   } else {
@@ -882,11 +890,9 @@ int launch_vq(const float* z, int64_t R, int Q, const float* w_in, const float* 
 // An id outside [0, n_codes) is an ERROR, as `codebook[idx]` is in the reference (vector_quantize_pytorch.py:310-314 raises /
 // device-asserts): the row is poisoned with NaN and counted in *bad_ids, which the engine reports (selftok_id_errors; the
 // host-buffer entry points return SELFTOK_ERR_BAD_ARG).  Nothing is clamped silently.
-__global__ void lookup_ln3_kernel(const int64_t* __restrict__ ids, int64_t R, const float* __restrict__ codebook,
-                                  int n_codes, int dim, const float* __restrict__ ln_w, const float* __restrict__ ln_b,
-                                  float* __restrict__ outs_q, int* __restrict__ bad_ids) {
-  const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (row >= R) return;
+__device__ __forceinline__ void lookup_ln3_row(int64_t row, const int64_t* __restrict__ ids, const float* __restrict__ codebook,
+                                               int n_codes, int dim, const float* __restrict__ ln_w, const float* __restrict__ ln_b,
+                                               float* __restrict__ outs_q, int* __restrict__ bad_ids) {
   const int64_t id = ids[row];
   if (id < 0 || id >= n_codes) {
     if (bad_ids) atomicAdd(bad_ids, 1);
@@ -901,11 +907,42 @@ __global__ void lookup_ln3_kernel(const int64_t* __restrict__ ids, int64_t R, co
   const float rstd = rsqrtf(var / (float)dim + 1e-6f);
   for (int d = 0; d < dim; ++d) outs_q[row * dim + d] = (codebook[id * dim + d] - mean) * rstd * ln_w[d] + ln_b[d];
 }
+__global__ void lookup_ln3_kernel(const int64_t* __restrict__ ids, int64_t R, const float* __restrict__ codebook,
+                                  int n_codes, int dim, const float* __restrict__ ln_w, const float* __restrict__ ln_b,
+                                  float* __restrict__ outs_q, int* __restrict__ bad_ids) {
+  const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (row >= R) return;
+  lookup_ln3_row(row, ids, codebook, n_codes, dim, ln_w, ln_b, outs_q, bad_ids);
+}
+// Positions >= n_tok[b] get zero rows (the padding of the reference's cut_of_k branch, rectified_flow.py:217-225): they are
+// masked as keys downstream, and their K / V rows must stay finite because a masked key still enters P V with P = 0.
+__global__ void lookup_ln3_prefix_kernel(const int64_t* __restrict__ ids, int B, int K, const int32_t* __restrict__ n_tok,
+                                         const float* __restrict__ codebook, int n_codes, int dim, const float* __restrict__ ln_w,
+                                         const float* __restrict__ ln_b, float* __restrict__ outs_q, int* __restrict__ bad_ids) {
+  const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (row >= (int64_t)B * K) return;
+  if ((int)(row % K) >= n_tok[row / K]) {
+    for (int d = 0; d < dim; ++d) outs_q[row * dim + d] = 0.f;
+    return;
+  }
+  lookup_ln3_row(row, ids, codebook, n_codes, dim, ln_w, ln_b, outs_q, bad_ids);
+}
 
 int launch_lookup_ln3(const int64_t* ids, int64_t R, const float* codebook, int n_codes, int code_dim,
                       const float* ln_w, const float* ln_b, float* outs_q, int* bad_ids, cudaStream_t s) {
   STK_CHECK(ids && codebook && ln_w && ln_b && outs_q && R > 0, -1, "lookup: bad arguments");
   lookup_ln3_kernel<<<(unsigned)((R + 127) / 128), 128, 0, s>>>(ids, R, codebook, n_codes, code_dim, ln_w, ln_b, outs_q, bad_ids);
+  count_launch();
+  STK_CUDA(cudaGetLastError());
+  return 0;
+}
+
+int launch_lookup_ln3_prefix(const int64_t* ids, int B, int K, const int32_t* n_tok, const float* codebook, int n_codes,
+                             int code_dim, const float* ln_w, const float* ln_b, float* outs_q, int* bad_ids, cudaStream_t s) {
+  STK_CHECK(ids && n_tok && codebook && ln_w && ln_b && outs_q && B > 0 && K > 0, -1, "lookup_prefix: bad arguments");
+  const int64_t R = (int64_t)B * K;
+  lookup_ln3_prefix_kernel<<<(unsigned)((R + 127) / 128), 128, 0, s>>>(ids, B, K, n_tok, codebook, n_codes, code_dim, ln_w, ln_b,
+                                                                       outs_q, bad_ids);
   count_launch();
   STK_CUDA(cudaGetLastError());
   return 0;

@@ -262,20 +262,23 @@ class SelftokPipeline:
         return self.engine.encode(x_0)
 
     @torch.no_grad()
-    def decode_latents(self, idx, noise: Optional[torch.Tensor] = None, cfg_scale: Optional[float] = None) -> torch.Tensor:
+    def decode_latents(self, idx, noise: Optional[torch.Tensor] = None, cfg_scale: Optional[float] = None, *,
+                       n_tokens=None) -> torch.Tensor:
         """tokens -> pred_x0 latents after the 50-step Euler loop.  `noise` defaults to the reference's draw:
         torch.randn on the CPU global generator, then moved to the device (SelftokPipeline.py:262-264).
         cfg_scale (None / 1: plain sampler): classifier-free guidance as RectifiedFlow.sample_one_step implements it
-        (rectified_flow.py:280-289) -- an explicit argument here because the reference pipeline never forwards its own."""
+        (rectified_flow.py:280-289) -- an explicit argument here because the reference pipeline never forwards its own.
+        n_tokens (an int, or one value per image in [1, K]): decode image b from its first n_tokens[b] tokens only, as
+        p_sample_loop(..., super_mask = arange(K) < n) does (rectified_flow.py:227-228); later ids are never read."""
         token_idx = torch.from_numpy(idx) if isinstance(idx, np.ndarray) else idx
         B = token_idx.shape[0]
         latent_dim = self.datasize // 8
         if noise is None:
             noise = torch.randn(B, self.dims.in_channels, latent_dim, latent_dim)
         if cfg_scale is None or float(cfg_scale) == 1.0:
-            out = self.engine.decode(token_idx, noise)
+            out = self.engine.decode(token_idx, noise, n_tokens=n_tokens)
         else:
-            out = self.engine.decode_cfg(token_idx, noise, float(cfg_scale))
+            out = self.engine.decode_cfg(token_idx, noise, float(cfg_scale), n_tokens=n_tokens)
         self._raise_on_bad_ids(token_idx)
         return out
 
@@ -286,9 +289,10 @@ class SelftokPipeline:
             raise IndexError("token id out of range for the codebook")
 
     @torch.no_grad()
-    def render_latents(self, idx) -> torch.Tensor:
+    def render_latents(self, idx, *, n_tokens=None) -> torch.Tensor:
+        """n_tokens: render image b from its first n_tokens[b] tokens (MMDiT_Renderer.forward(..., mask=...), sd3/mmdit.py:1529)."""
         token_idx = torch.from_numpy(idx) if isinstance(idx, np.ndarray) else idx
-        out = self.engine.render(token_idx)
+        out = self.engine.render(token_idx, n_tokens=n_tokens)
         self._raise_on_bad_ids(token_idx)
         return out
 
@@ -336,10 +340,10 @@ class SelftokPipeline:
         return tokens
 
     @torch.no_grad()
-    def decoding(self, idx, device):
+    def decoding(self, idx, device, *, n_tokens=None):
         print("Begin decoding.")
         self._need_vae()
-        pred_x0 = self.decode_latents(idx)
+        pred_x0 = self.decode_latents(idx, n_tokens=n_tokens)
         pred_x0_out = SD3LatentFormat().process_out(pred_x0).to(self.dtype)
         recons = self.vae.decode(pred_x0_out, return_dict=False)[0]
         norm_ip(recons, -1, 1)
@@ -347,19 +351,19 @@ class SelftokPipeline:
         return recons
 
     @torch.no_grad()
-    def decoding_cfg(self, idx, device, cfg_scale: Optional[float] = None):
+    def decoding_cfg(self, idx, device, cfg_scale: Optional[float] = None, *, n_tokens=None):
         """decoding() with the guided sampler (cfg_scale defaults to the constructor's)."""
         self._need_vae()
-        pred_x0 = self.decode_latents(idx, cfg_scale=self.cfg_scale if cfg_scale is None else cfg_scale)
+        pred_x0 = self.decode_latents(idx, cfg_scale=self.cfg_scale if cfg_scale is None else cfg_scale, n_tokens=n_tokens)
         recons = self.vae.decode(SD3LatentFormat().process_out(pred_x0).to(self.dtype), return_dict=False)[0]
         norm_ip(recons, -1, 1)
         return recons
 
     @torch.no_grad()
-    def decoding_with_renderer(self, idx, device):
+    def decoding_with_renderer(self, idx, device, *, n_tokens=None):
         print("Begin decoding with Renderer.")
         self._need_vae()
-        pred_x0 = self.render_latents(idx)
+        pred_x0 = self.render_latents(idx, n_tokens=n_tokens)
         pred_x0_out = SD3LatentFormat().process_out(pred_x0).to(self.dtype)
         recons = self.vae.decode(pred_x0_out)[0]
         norm_ip(recons, -1, 1)
